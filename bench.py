@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric (GICP scans/sec) on BASELINE.json's configs.
 
-    python bench.py [--config c2|c3|c4|c5] [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--config c2|c3|c4|c5] [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 --config c2 (default, BASELINE configs[1], the configuration the metric is quoted on): scan-to-scan odometry.
     A synthetic 64-beam stream of 100 scans, 131072 rays each (tools/gen_lidar.py); per scan
@@ -32,6 +32,12 @@
     roofline object is the NN-search kernel (the HBM-bound kernel of this path) on the scan's 200k queries.
 --impl reference: the CPU arm = oracle/ (C port of the reference; the reference itself needs PCL/ROS and cannot be
     built here), all host threads, the same config, each step a bounded sample of the b200 arm's step (one scan).
+--dump-outputs DIR: after the timed steps, what the headline arm returned in its LAST timed step, as DIR/<name>.npy
+    (float32 / float64; rank 0's stream).  c2: per scan of the step, the pipeline's pose and align result
+    (final_transformation, converged, iterations, n_correspondences, delta, n_filtered); c3-c5: the same for the step's
+    one scan plus its filtered cloud (filtered_cloud, x y z intensity).  The inputs are generated from fixed seeds and
+    the step's scans depend only on the arguments, so two builds run with the same arguments can be compared output
+    for output.
 
 N>1 (torchrun): one independent scan stream per GPU (weak scaling, no data-path collective); barrier + device sync
 on both sides of the timed region, max over ranks.
@@ -86,7 +92,13 @@ def parse():
     ap.add_argument("--stream-scans", type=int, default=0, help="distinct scans of the stream (0 = the config's; profiling aid)")
     ap.add_argument("--profile", action="store_true",
                     help="profiling aid for ncu: the blocking per-scan calls only (no pipeline, no e2e arm, no CPU baseline)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step as DIR/<name>.npy "
+                         "(c2: the pipeline's results for the step's scans; c3-c5: the align result and the filtered scan)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.profile):
+        ap.error("--dump-outputs writes the outputs of the b200 arm's timed path (not with --impl reference or --profile)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------ helpers
@@ -658,6 +670,25 @@ def pose_deltas(cpu_poses, gpu_poses, spread=None):
     return out
 
 
+def gicp_outputs(results, n_filtered):
+    """what lb_gicp_align returns to its caller for each scan of a step (timings left out: they are not results)"""
+    return {"final_transformation": np.array([list(r.final_transformation) for r in results], dtype=np.float32).reshape(-1, 4, 4),
+            "converged": np.array([r.converged for r in results], dtype=np.float64),
+            "iterations": np.array([r.iterations for r in results], dtype=np.float64),
+            "n_correspondences": np.array([r.n_correspondences for r in results], dtype=np.float64),
+            "delta": np.array([r.delta for r in results], dtype=np.float64),
+            "n_filtered": np.array(n_filtered, dtype=np.float64)}
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: one float32 / float64 array per file, DIR/<name>.npy.  The largest is one filtered scan
+    (c5: ~200k points x 4 floats), far below 64 MB in all."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------ c2
 def run_c2(ctx):
     args, cfg, workload, torch, L, lb, api = ctx.args, ctx.cfg, ctx.workload, ctx.torch, ctx.L, ctx.lb, ctx.api
@@ -824,6 +855,9 @@ def run_c2(ctx):
     k_n = sum(n for _, n in kt)
     k_ms = sum(ms * n for ms, n in kt) / k_n if k_n else 0.0
     pipe_same, pipe_compared = equals_sequential(p_out)      # same scans, same kernels: bit-identical poses expected
+    if args.dump_outputs and ctx.rank == 0:                   # p_out is in submission order: the last step's scans are last
+        last = p_out[-args.scans_per_step:]
+        dump_outputs(args.dump_outputs, gicp_outputs([r.gicp for r in last], [r.n_filtered for r in last]))
     e2e_ms, e_out, _ = pipelined_run(odo, submit_host, n_scans, n_warm)
     e2e_h2d = args.scans_per_step * nraw * POINT_STEP
     e2e_d2h = args.scans_per_step * (int(np.mean([r.n_filtered for r in e_out])) * POINT_STEP + C.sizeof(api.OdometryResult))
@@ -1009,6 +1043,11 @@ def run_submap(ctx):
     gicp.resetKernelTimes(False)
     dev_ms, wall, launches, _ = arm(False, False, n_timed, warm)
     clocks = sampler.stop()
+    if args.dump_outputs and ctx.rank == 0:      # res, n_out and d_filt[0] still hold the last timed scan's results
+        n = n_out.value
+        cloud = ctx.d_filt[0][:n * POINT_STEP].cpu().numpy().view(np.float32).reshape(n, POINT_STEP // 4)
+        dump_outputs(args.dump_outputs, dict(gicp_outputs([res], [n]),
+                                             filtered_cloud=np.ascontiguousarray(cloud[:, [0, 1, 2, 4]])))   # x y z intensity
     gpu_poses = list(state["poses"])
     iters = np.array(state["iters"], dtype=np.float64); evals = np.array(state["evals"], dtype=np.float64)
     ncorr = np.array(state["ncorr"], dtype=np.float64); nsrc = np.array(state["nsrc"], dtype=np.float64)

@@ -1,13 +1,15 @@
 """Convert the reference's GICP test clouds (multithreaded_gicp/test/*_82_garage.pcd,
 binary PCD, fields x y z intensity float32) into tests/golden/garage.npz.
 
-Run in the authoring container only (needs /root/reference); the .npz is committed
-because /root/reference does not exist on the GPU box.
+    python tests/golden/make_garage_fixture.py <LOCUS checkout>
+
+Needs a checkout of the original LOCUS project; the .npz is committed so that the
+tests do not.
 """
 import os
-import numpy as np
+import sys
 
-REF = "/root/reference/multithreaded_gicp/test"
+import numpy as np
 
 
 def read_pcd(path):
@@ -21,8 +23,11 @@ def read_pcd(path):
 
 
 if __name__ == "__main__":
-    q = read_pcd(os.path.join(REF, "query_82_garage.pcd"))
-    r = read_pcd(os.path.join(REF, "reference_82_garage.pcd"))
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    ref = os.path.join(sys.argv[1], "multithreaded_gicp", "test")
+    q = read_pcd(os.path.join(ref, "query_82_garage.pcd"))
+    r = read_pcd(os.path.join(ref, "reference_82_garage.pcd"))
     assert q.shape == (811, 4) and r.shape == (8112, 4)
     out = os.path.join(os.path.dirname(os.path.abspath(__file__)), "garage.npz")
     np.savez_compressed(out, query=q, reference=r)

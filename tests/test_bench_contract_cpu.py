@@ -45,6 +45,14 @@ def test_reference_arm_under_torchrun_rank0_only():
     _check(lines[0], 2)
 
 
+def test_dump_outputs_refused_without_the_b200_arm(tmp_path):
+    """--dump-outputs writes what the b200 arm's timed path returned; the CPU arm refuses it instead of ignoring it"""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                       stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not r.stdout.strip()
+    assert os.listdir(tmp_path) == []
+
+
 def test_reference_arm_c3_contract_line():
     """--config c3 (scan-to-submap, BASELINE configs[2]): same contract line; the CPU arm keeps the submap's kd-tree and
     covariances between scans, like the reference does while setInputTarget is not called again"""
